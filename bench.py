@@ -61,7 +61,12 @@ def parse():
     ap.add_argument("--frames", default="person", choices=["person", "noise", "const"], help="synthetic stream kind (SURVEY 8d)")
     ap.add_argument("--launches-per-step", type=int, default=20, help="graph launches per stream per timed step (lengthens the timed window)")
     ap.add_argument("--tune", action="append", default=[], metavar="NAME=VALUE", help="bsb_set_tuning switch (A/B runs): pw_variant, dw_plane, post_tma, ...")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step (a seeded sample of pixels) to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs records the outputs of the b200 path only")
+    return args
 
 
 def dist_env():
@@ -316,7 +321,30 @@ def post_bytes(W, H, ow, oh, B, yuyv_in, bg_per_frame, bg_cache):
     return B * per_frame + (B * bg if bg_per_frame else bg)
 
 
-def measure(args, wl, key, dev, rank, world, S, B, steps, warmup, lps, with_e2e, with_clocks, kind="person"):
+DUMP_PIXELS = 1 << 20        # sampled pixels of --dump-outputs: 6 float32 values + 1 float64 index each, 32 MB in all
+
+
+def dump_outputs(path, slots, B, H, W):
+    """--dump-outputs: what one step returned to its caller (RGB composite, YUYV frame and mask of every stream's batch),
+    `slots` holding one ring slot per stream, written as float32 for a fixed, seeded sample of DUMP_PIXELS pixels (all
+    pixels if there are fewer).  pixel_index.npy holds each sample's flat index into [stream, frame, y, x]."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    per = B * H * W
+    total = len(slots) * per
+    idx = np.arange(total) if total <= DUMP_PIXELS else np.unique(np.random.default_rng(0).integers(0, total, DUMP_PIXELS))
+    parts = {"composite": [], "yuyv": [], "mask": []}
+    for s, sl in enumerate(slots):
+        sel = torch.from_numpy(idx[(idx >= s * per) & (idx < (s + 1) * per)] - s * per).to(sl["d_out"].device)
+        parts["composite"].append(sl["d_out"].view(per, 3)[sel])
+        parts["yuyv"].append(sl["d_yuyv"].view(per, 2)[sel])
+        parts["mask"].append(sl["d_mask"].view(per)[sel])
+    for name, p in parts.items():
+        np.save(os.path.join(path, name + ".npy"), torch.cat(p).cpu().numpy().astype(np.float32))
+    np.save(os.path.join(path, "pixel_index.npy"), idx.astype(np.float64))
+
+
+def measure(args, wl, key, dev, rank, world, S, B, steps, warmup, lps, with_e2e, with_clocks, kind="person", dump_dir=None):
     """One workload on this rank's GPU: device-resident throughput, optional end-to-end, per-stage times, rooflines."""
     import torch
 
@@ -385,6 +413,9 @@ def measure(args, wl, key, dev, rank, world, S, B, steps, warmup, lps, with_e2e,
         e.record(s)
     barrier()
     ms = max(ev0.elapsed_time(e) for e in ev1)
+    if dump_dir:
+        last = ((warmup + steps) * lps - 1) % R            # ring slot written by the last launch of the last timed step
+        dump_outputs(dump_dir, [rg["slots"][last] for rg in rings], B, H, W)
     frames_total, secs, value = sharding.reduce_throughput(S * B * lps * steps, ms * 1e-3,
                                                             torch.distributed if world > 1 else None, f"cuda:{dev}")
     ms = secs * 1e3
@@ -597,7 +628,8 @@ def run_b200(args, wl):
         bs.set_tuning(name, int(val))
     S, B = args.streams or wl.get("streams", 8), args.batch or wl.get("batch", 32)
     lps = max(1, args.launches_per_step)
-    m = measure(args, wl, args.workload, dev, rank, world, S, B, args.steps, args.warmup, lps, not args.no_e2e, True, kind=args.frames)
+    m = measure(args, wl, args.workload, dev, rank, world, S, B, args.steps, args.warmup, lps, not args.no_e2e, True, kind=args.frames,
+                dump_dir=args.dump_outputs if rank == 0 else None)
 
     # ---- the other BASELINE configs, short runs on one GPU (N = 1 only): parsed.configs ----
     configs = None

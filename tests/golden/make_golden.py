@@ -1,19 +1,27 @@
-"""Generate the committed golden fixtures (run in the build container, where cv2 4.13
-and /root/reference exist):
+"""Generate the committed golden fixtures (needs cv2 4.13, and a checkout of the original
+backscrub tree: oracle/_ref built from it for tconv_ref_golden.npz, its path in
+BACKSCRUB_REFERENCE for reference_header_symbols.txt):
 
   image_ops_golden.npz   cv2 outputs for small seeded inputs (resize/blur/RGB2YUV/
                          bilateral/convertTo) — pins the oracle's image primitives on
                          boxes whose cv2 build may differ.
   tconv_ref_golden.npz   outputs of the REFERENCE's lib/transpose_conv_bias.cc
-                         (oracle/_ref) for seeded inputs — travels to the GPU box.
+                         (oracle/_ref) for seeded inputs, including the cases and the
+                         known answer of tests/test_oracle_nn.py.
   model_torch_golden.npz torch-fp64 evaluation of each .tflite on one synthetic input:
                          decision bitmap + output statistics.
   pipeline_golden.npz    oracle regression outputs (mask bits, composite checksums).
+  reference_header_symbols.txt
+                         mangled names of the C++-linkage functions that tests/cpp/dropin_test.cc
+                         needs when compiled against the REFERENCE's own lib/libbackscrub.h and
+                         app/background.h (include order of its CMakeLists.txt:72).
 
     python tests/golden/make_golden.py
 """
 import os
+import subprocess
 import sys
+import tempfile
 
 import cv2
 import numpy as np
@@ -25,6 +33,7 @@ from tests import synth, torch_graph  # noqa: E402
 from tests.conftest import MODELS, model_path  # noqa: E402
 
 OUT = os.path.dirname(os.path.abspath(__file__))
+TCONV_CASES = [(8, 8, 16, 1), (5, 7, 16, 2), (3, 3, 4, 3)]
 
 
 def image_ops():
@@ -69,6 +78,17 @@ def tconv_ref():
         w = rng.standard_normal((oc, 2, 2, ic)).astype(np.float32)
         b = rng.standard_normal(oc).astype(np.float32)
         d[f"x{i}"], d[f"w{i}"], d[f"b{i}"], d[f"y{i}"] = x, w, b, po.ref_tconv_bias(x, w, b)
+    # the cases of tests/test_oracle_nn.py, which compare the oracle with these stored outputs
+    for ih, iw, ic, oc in TCONV_CASES:
+        rng = np.random.default_rng(ih * 100 + oc)
+        x = rng.standard_normal((ih, iw, ic)).astype(np.float32)
+        w = rng.standard_normal((oc, 2, 2, ic)).astype(np.float32)
+        b = rng.standard_normal(oc).astype(np.float32)
+        key = "case_%dx%dx%dx%d" % (ih, iw, ic, oc)
+        d[key + "_x"], d[key + "_w"], d[key + "_b"], d[key + "_y"] = x, w, b, po.ref_tconv_bias(x, w, b)
+    x = np.array([1, 2, 3, 4], np.float32).reshape(2, 2, 1)
+    w = np.array([1, 10, 100, 1000], np.float32).reshape(1, 2, 2, 1)
+    d["kat_y"] = po.ref_tconv_bias(x, w, [0.5])
     np.savez_compressed(os.path.join(OUT, "tconv_ref_golden.npz"), **d)
 
 
@@ -120,7 +140,24 @@ def model_cv2dnn():
                         mlkit_decision=np.packbits(out > 0.65), mlkit_margin_ok=np.packbits(np.abs(out - 0.65) > 1e-3))
 
 
+def reference_header_symbols():
+    ref = os.environ.get("BACKSCRUB_REFERENCE")
+    if not ref:
+        print("BACKSCRUB_REFERENCE not set; skipping reference_header_symbols")
+        return
+    cpp = os.path.join(ROOT, "tests", "cpp")
+    with tempfile.TemporaryDirectory() as tmp:
+        obj = os.path.join(tmp, "dropin_test_ref.o")
+        subprocess.check_call(["g++", "-std=c++17", "-O1", "-c", "-I" + os.path.join(cpp, "stub"), "-I" + ref, "-I" + os.path.join(ref, "app"),
+                               "-I" + os.path.join(ROOT, "include"), "-o", obj, os.path.join(cpp, "dropin_test.cc")])
+        undef = [ln.split()[-1] for ln in subprocess.run(["nm", "-u", obj], capture_output=True, text=True, check=True).stdout.splitlines()]
+    names = subprocess.run(["c++filt"], input="\n".join(undef), capture_output=True, text=True, check=True).stdout.splitlines()
+    keep = sorted(m for m, d in zip(undef, names) if d.startswith(("bs_", "load_background(", "grab_background(", "grab_thumbnail(")))
+    with open(os.path.join(OUT, "reference_header_symbols.txt"), "w") as f:
+        f.write("\n".join(keep) + "\n")
+
+
 if __name__ == "__main__":
-    image_ops(); tconv_ref(); model_torch(); pipeline(); model_cv2dnn()
+    image_ops(); tconv_ref(); model_torch(); pipeline(); model_cv2dnn(); reference_header_symbols()
     for f in sorted(os.listdir(OUT)):
         print(f, os.path.getsize(os.path.join(OUT, f)))

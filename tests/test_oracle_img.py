@@ -1,11 +1,14 @@
 """Oracle 8-bit image primitives vs the in-container cv2 (the live golden; OpenCV is
 a system dependency of the reference, SURVEY.md §8c / Appendix B) and vs literal
 formulas for the app/deepseg.cc helpers."""
+import os
+
 import cv2
 import numpy as np
 import pytest
 
 from oracle import pyoracle as po
+from tests.conftest import ROOT
 
 RNG = np.random.default_rng(42)
 
@@ -100,7 +103,7 @@ def test_bilateral_vs_cv2(w, h):
     """cv::bilateralFilter(5,100,100).  OpenCV's own code paths (IPP / AVX2+FMA / SSE
     baseline) already disagree with one another on a few pixels per image by 1 LSB
     (float summation order), so the pin is: max |diff| <= 1 and <= 1e-4 of the values."""
-    img = cv2.imread("backgrounds/screenshot.jpg")
+    img = cv2.imread(os.path.join(ROOT, "backgrounds", "screenshot.jpg"))
     srcs = [cv2.resize(img[:, :640], (w, h)), RNG.integers(0, 256, (h, w, 3), dtype=np.uint8)]
     for src in srcs:
         got = po.bilateral_d5(src).astype(int)

@@ -4,15 +4,19 @@ Vectors transcribed (as data) from the vendored TFLite tests the survey lists
 (§4, §8c): kernels/conv_test.cc, depthwise_conv_test.cc, pooling_test.cc,
 resize_bilinear_test.cc, activations_test.cc, transpose_conv_test.cc,
 fully_connected_test.cc — tolerance ArrayFloatNear 1e-5 (kernels/test_util.h:56-57).
-Also pins or_tconv_bias against oracle/_ref (the reference's own
-lib/transpose_conv_bias.cc compiled in place).
+Also pins or_tconv_bias against the stored outputs of the reference's own
+lib/transpose_conv_bias.cc (tests/golden/tconv_ref_golden.npz).
 """
+import os
+
 import numpy as np
 import pytest
 
 from oracle import pyoracle as po
+from tests.conftest import ROOT
 
 TOL = 1e-5
+TCONV_REF_GOLDEN = os.path.join(ROOT, "tests", "golden", "tconv_ref_golden.npz")
 
 
 def near(a, b, tol=TOL):
@@ -229,30 +233,27 @@ def test_tconv_survey_known_answer():  # SURVEY.md §8c (probe of the compiled r
     near(po.tconv_bias(x, w, [0.5]), exp)
 
 
-@pytest.mark.skipif(po.ref_tconv_lib() is None, reason="oracle/_ref not built (no /root/reference here)")
 @pytest.mark.parametrize("shape", [(8, 8, 16, 1), (5, 7, 16, 2), (3, 3, 4, 3)])
 def test_tconv_matches_compiled_reference(shape):
     """or_tconv_bias vs the reference's own lib/transpose_conv_bias.cc (k2 s2 SAME, the
-    MLKit/Meet configuration).  The reference accumulates `+= a*b` (compiler-dependent
-    contraction) and the oracle uses fmaf, so the bound is a few ulp, not bit equality."""
+    MLKit/Meet configuration), whose outputs on these seeded inputs are stored in
+    tests/golden/tconv_ref_golden.npz (tests/golden/make_golden.py).  The reference accumulates
+    `+= a*b` (compiler-dependent contraction) and the oracle uses fmaf, so the bound is a few
+    ulp, not bit equality."""
     ih, iw, ic, oc = shape
-    rng = np.random.default_rng(ih * 100 + oc)
-    x = rng.standard_normal((ih, iw, ic)).astype(np.float32)
-    w = rng.standard_normal((oc, 2, 2, ic)).astype(np.float32)
-    b = rng.standard_normal(oc).astype(np.float32)
-    ref = po.ref_tconv_bias(x, w, b)
+    z = np.load(TCONV_REF_GOLDEN)
+    key = "case_%dx%dx%dx%d" % shape
+    x, w, b, ref = z[key + "_x"], z[key + "_w"], z[key + "_b"], z[key + "_y"]
     got = po.tconv_bias(x, w, b)
     # lib/transpose_conv_bias.cc:157-184: SAME trims (k - (in-1)%stride - 1) -> 2*in for even, 2*in-1 for odd sizes
     assert ref.shape == got.shape == (2 * ih - ih % 2, 2 * iw - iw % 2, oc)
     np.testing.assert_allclose(got, ref, rtol=3e-6, atol=3e-6)
 
 
-@pytest.mark.skipif(po.ref_tconv_lib() is None, reason="oracle/_ref not built")
 def test_ref_tconv_known_answer():
-    x = np.array([1, 2, 3, 4], np.float32).reshape(2, 2, 1)
-    w = np.array([1, 10, 100, 1000], np.float32).reshape(1, 2, 2, 1)
+    """The stored output of the compiled reference op on the survey's known-answer input."""
     exp = [1.5, 10.5, 2.5, 20.5, 100.5, 1000.5, 200.5, 2000.5, 3.5, 30.5, 4.5, 40.5, 300.5, 3000.5, 400.5, 4000.5]
-    near(po.ref_tconv_bias(x, w, [0.5]), exp)
+    near(np.load(TCONV_REF_GOLDEN)["kat_y"], exp)
 
 
 def test_same_padding_rules():  # kernels/padding.h:23-82; SURVEY Appendix A closed forms
